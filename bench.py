@@ -3,6 +3,7 @@
 imm_ukf_jpda) on B200, next to the reference's own CPU implementation timed on the same host.
 
     python bench.py [--gpus N] [--steps K] [--warmup W]           # our CUDA path
+    python bench.py ... --dump-outputs DIR                        # + the last timed step's boxes and live tracks as DIR/*.npy
     python bench.py --impl reference [--steps K] [--warmup W]     # the reference's sources (oracle/_ref) on the host CPU
     torchrun ... bench.py --gpus N ...                            # one rank per GPU, independent sensor streams (weak scaling)
 
@@ -20,8 +21,9 @@ Printed JSON (rank 0, one line):
   cpu_baseline  the reference's own four entry points on a bounded sample of the same frames, one host thread
   parity_check  the CUDA path against the reference ON THE BENCH SCENE, frame by frame over the cpu_baseline sample: counts, boxes
             (bit-exact), trackManage (identical), UKF states of well-conditioned tracks (<= 1e-4); a failing check withholds `value`
-  windows   the K-step timed region is repeated `windows` times on consecutive frames (barrier + synchronize on both sides of
-            each); `value`, `ms_per_step` and `e2e` are the MEDIAN window, `window_values` lists all of them
+  windows   --windows R repeats the K-step timed region R times on consecutive frames (default 1, so exactly K steps are timed;
+            barrier + synchronize on both sides of each); `value`, `ms_per_step` and `e2e` are the MEDIAN window, `window_values`
+            lists all of them
   latency_us    p50 / p99 per stage and per frame, one frame in flight (CUDA events) and at the pipeline's depth (host clock)
   batched_8x120k  BASELINE.json configs[3]: 8 sensor streams, one frame each per tick, one shared track table: ticks through
             lmot_batch_dev, and the ground_removal + CCL roofline of the two batched launches
@@ -511,12 +513,30 @@ def batched_block(lmot, synth, local_rank, stream, peak, ticks=12, warm=3, F=8):
 
 
 # ------------------------------------------------------------------------------------------- our arm
+PER_TRACK = ("targets", "vandyaw", "track_manage", "is_static", "is_vis")
+
+
+def dump_outputs(out_dir, res):
+    """One .npy per array of a frame result: float32 data as is, integer and flag arrays widened to float64 (exact).
+    Per-track arrays keep the live tracks (trackManage != 0) and `track_index` gives their rows in the table: a dead
+    slot stays in the append-only table with whatever state its filter ended in (NaN when it diverged, as in the
+    reference), and the tracking node publishes only live tracks."""
+    os.makedirs(out_dir, exist_ok=True)
+    live = np.asarray(res["track_manage"]) != 0
+    out = {**res, "track_index": np.flatnonzero(live)}
+    for name, v in out.items():
+        a = np.asarray(v)
+        a = a[live] if name in PER_TRACK else a
+        a = a if a.dtype in (np.float32, np.float64) else a.astype(np.float64)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=200)
     ap.add_argument("--warmup", type=int, default=20)
-    ap.add_argument("--windows", type=int, default=0, help="repetitions of the K-step timed window (0 = auto: 5 for short runs, 1 from K = 200)")
+    ap.add_argument("--windows", type=int, default=1, help="repetitions of the K-step timed window (each one times K more steps)")
     ap.add_argument("--impl", default="lmot", choices=["lmot", "reference"])
     ap.add_argument("--cpu-sample", type=int, default=60, help="frames of the CPU baseline / parity sample (rank 0, N=1)")
     ap.add_argument("--tracker-stress", type=int, default=40, help="timed steps of the 1024x256 tracker-only workload (0 = skip; rank 0, N=1)")
@@ -528,6 +548,8 @@ def main():
                     help="N>1 only: all ranks feed ONE track table (NCCL all_gather of boxes, tracker on rank 0, NCCL broadcast of the "
                          "outputs and of the table): 'streams' = N sensors per tick (configs[3]), 'frames' = one sensor, frames sharded "
                          "round-robin over the ranks (configs[4]).  Default: N independent streams, no collective.")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (boxes and live tracks, rank 0) to DIR/<name>.npy, float32 / float64")
     args = ap.parse_args()
 
     rank = int(os.environ.get("RANK", "0"))
@@ -549,7 +571,7 @@ def main():
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
     lmot = importlib.import_module(PKG)
     K, W = args.steps, max(args.warmup, 3)
-    R = args.windows if args.windows > 0 else max(1, min(5, 200 // max(K, 1)))
+    R = max(1, args.windows)
 
     # ---- inputs: W + R*K consecutive frames of this rank's sensor stream, resident in HBM and in pinned host memory
     ts, frames = make_frames(synth, W + R * K, seed_offset=rank)
@@ -607,6 +629,8 @@ def main():
         win_ms.append(e0.elapsed_time(e1))
     res_dev = ctx.frame_fetch()
     live_tracks = int((res_dev["track_manage"] > 0).sum())
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, res_dev)
 
     # ---- (2) per-stage device time of the same frames, ONE frame in flight (CUDA events on the launching stream)
     ctx.tracker_reset()

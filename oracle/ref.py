@@ -169,8 +169,8 @@ class RefOracle(_OracleBase):
 
 
 class PortOracle(_OracleBase):
-    def __init__(self, mode: str = "intended"):
-        super().__init__(os.path.join(HERE, "liboracle_port.so"), "port_")
+    def __init__(self, mode: str = "intended", path: str | None = None):
+        super().__init__(path or os.path.join(HERE, "liboracle_port.so"), "port_")
         self.mode = mode
         self.lib.port_set_rule_mode(0 if mode == "intended" else 1)
 

@@ -6,7 +6,17 @@ MAR contract (oracle/mar_contract.cpp) in both ruleBasedFilter modes; markers (v
 import numpy as np
 import pytest
 
+from oracle.recorded import ReferenceDigest
+
 pytestmark = pytest.mark.gpu
+
+
+def _bit_equal(a, ref):
+    """bit-exact equality with a reference result (the large ones are stored as a digest, oracle/recorded.py)"""
+    if isinstance(ref, ReferenceDigest):
+        return ref.matches(a)
+    a = np.ascontiguousarray(a, ref.dtype)
+    return a.shape == ref.shape and np.array_equal(a.view(f"u{a.dtype.itemsize}"), np.ascontiguousarray(ref).view(f"u{a.dtype.itemsize}"))
 
 
 def _elevated(ref, pts):
@@ -148,10 +158,11 @@ def test_cluster_node_side_outputs_bit_exact(lm, ref_intended, synth):
             g, k = lm.component_cluster(e)
             assert k == k_ref and np.array_equal(g, g_ref)
             cl, ob, cm = lm.cluster_outputs()
-            assert cl.shape[0] == cl_r.shape[0] and np.array_equal(cl[:, :3].view(np.uint32), cl_r.view(np.uint32))
+            assert cl.shape[0] == cl_r.shape[0] and _bit_equal(cl[:, :3], cl_r)
             assert ob.shape[0] == ob_r.shape[0] and ob.shape[0] > 100
-            assert np.array_equal(ob[:, :3].astype(np.float64), ob_r[:, :3]) and np.array_equal(ob[:, 3].astype(np.int64), ob_r[:, 3].astype(np.int64))
-            assert np.array_equal(cm, cm_r) and cm.max() == 100
+            # [x, y, z, cluster id] in double, as setObsMsg writes them
+            assert _bit_equal(np.concatenate([ob[:, :3].astype(np.float64), ob[:, 3:].astype(np.int64).astype(np.float64)], 1), ob_r)
+            assert _bit_equal(cm, cm_r) and cm.max() == 100
     # twice in a row: the scratch grid is back at rest
     cl2, ob2, cm2 = lm.cluster_outputs()
     assert np.array_equal(cl2, cl) and np.array_equal(ob2, ob) and np.array_equal(cm2, cm)
